@@ -9,7 +9,13 @@ resident in HBM; `e2e` is the same iteration driven through the reference-facing
 pinned HOST buffers, host<->device copies inside the timed region.  Extra keys report 512^2 images/s
 (20 steps + VAE decode), the tensor-core roofline of the dominant kernel and the CPU baseline.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes, after the timed steps, what the timed paths computed in their last step as DIR/<name>.npy
+(float32): `latents` and `noise_pred` (the UNet output, rows uncond / cond) of the device loop, `e2e_latents` and
+`e2e_noise_pred` of the boundary loop, `image` (the last decoded image of the images/s loop); `noise_pred` alone
+for `--impl reference`.  All inputs derive from fixed seeds, so two builds run with the same arguments can be
+compared output for output.
 """
 import argparse
 import json
@@ -46,6 +52,15 @@ def _peaks():
             d = json.load(f)
         return d["bf16_tflops"], d["bf16_tflops_sustained"], d["hbm_gbs"], "measured"
     return 1590.0, 1400.0, 6650.0, "fallback"
+
+
+def dump_outputs(out_dir, arrays):
+    """DIR/<name>.npy in float32 for every array (a few MB in all; the bound keeps dumps comparable and small)."""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in arrays.items()}
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 class ClockSampler:
@@ -140,8 +155,8 @@ def time_cpu(budget_s=25.0, max_steps=3, warmup=1):
 
 def run_reference_arm(args, rank, world):
     """`--impl reference`: the reference's own CPU implementation of the path (its unmodified PyTorch-CPU UNet modules
-    when /root/reference is present, else the oracle restatement of them) on the box's host cores, same `config`,
-    metric and unit as the b200sd arm, EXACTLY --steps timed UNet forwards after --warmup untimed ones (a CPU
+    when $B200SD_REFERENCE names a reference checkout, else the oracle restatement of them) on the box's host cores,
+    same `config`, metric and unit as the b200sd arm, EXACTLY --steps timed UNet forwards after --warmup untimed ones (a CPU
     forward takes seconds: the default 40 + 3 finish within a few minutes).  Rank 0 only."""
     if rank != 0:
         return
@@ -151,8 +166,10 @@ def run_reference_arm(args, rank, world):
         fn()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        fn()
+        out = fn()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"noise_pred": out.numpy()})
     val = args.steps / dt
     line = {
         "impl": "reference", "metric": "diffusion_iter_per_s", "value": round(val, 4), "unit": "iter/s",
@@ -390,8 +407,14 @@ def run_gpu_arm(args, rank, local_rank, world):
     e1.record()
     barrier()
     ms_dev = e0.elapsed_time(e1)
+    outputs = {}
+    if args.dump_outputs and rank == 0:
+        outputs["latents"] = pipe._latents.cpu().numpy()
+        outputs["noise_pred"] = unet._out_nhwc.permute(0, 3, 1, 2).cpu().numpy()
     if args.quick:
         if rank == 0:
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, outputs)
             print(json.dumps({"quick": True, "iter_per_s": round(world * args.steps / (ms_dev * 1e-3), 2),
                               "ms_per_step": round(ms_dev / args.steps, 4), "launches_per_step": round(launches_per_step, 1),
                               "fused": os.environ.get("B200SD_FUSED", "ln"), "pdl": os.environ.get("B200SD_PDL", "1")}),
@@ -416,9 +439,11 @@ def run_gpu_arm(args, rank, local_rank, world):
         np_t[:] = float(st.timestep)
         out = unet(sample=np_sample, timestep=np_t, encoder_hidden_states=np_ctx)["noise_pred"]  # H2D + D2H inside
         eps = out[:1] + GUIDANCE * (out[1:] - out[:1])          # host CFG + DDIM exactly like pipeline.py:559-569
-        h_lat.copy_(torch.from_numpy(st.cx * h_lat.numpy() + st.ce * eps))
+        lat = st.cx * h_lat.numpy() + st.ce * eps
+        h_lat.copy_(torch.from_numpy(lat))
         if (i + 1) % N_STEPS_IMG == 0:
             h_lat.copy_(lat0.cpu())
+        return out, lat
 
     for i in range(3):
         e2e_step(i)
@@ -426,10 +451,12 @@ def run_gpu_arm(args, rank, local_rank, world):
     t0 = time.perf_counter()
     e0.record()
     for i in range(args.steps):
-        e2e_step(i)
+        last = e2e_step(i)
     e1.record()
     barrier()
     ms_e2e = max(e0.elapsed_time(e1), (time.perf_counter() - t0) * 1e3)
+    if outputs:
+        outputs["e2e_noise_pred"], outputs["e2e_latents"] = last
     clocks = sampler.stop()
 
     # ---- images/s: 20 steps + VAE decode through the public device-resident pipeline loop, >= 5 images ----
@@ -447,6 +474,8 @@ def run_gpu_arm(args, rank, local_rank, world):
     e1.record()
     barrier()
     ms_img = e0.elapsed_time(e1) / n_img
+    if outputs:
+        outputs["image"] = host_img.numpy()
 
     # ---- BASELINE configs[2] shape: 8 prompts per GPU (UNet batch 16), 20 steps + VAE decode of all 8 ----
     ms_b8 = float("nan")
@@ -526,6 +555,8 @@ def run_gpu_arm(args, rank, local_rank, world):
             "image_checksum": float(host_img.double().sum()),
         }
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.destroy_process_group()
 
@@ -541,6 +572,8 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the SDXL-768 / ControlNet configs (N = 1 only)")
     ap.add_argument("--profile-step", action="store_true",
                     help="run ONE eager denoising iteration between cudaProfilerStart/Stop (for ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's outputs as DIR/<name>.npy (float32)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -551,8 +584,7 @@ def main():
     if world == 1 and args.gpus > 1:
         # convenience: re-launch under torchrun
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}",
-               "--master-addr", "127.0.0.1", "--master-port", "29517", os.path.abspath(__file__), "--gpus",
-               str(args.gpus), "--steps", str(args.steps), "--warmup", str(args.warmup)]
+               "--master-addr", "127.0.0.1", "--master-port", "29517", os.path.abspath(__file__), *sys.argv[1:]]
         sys.exit(subprocess.call(cmd))
     if not torch.cuda.is_available():
         print(json.dumps({"error": "no CUDA device: b200sd has no CPU fallback; use --impl reference for the CPU arm"}))

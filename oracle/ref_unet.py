@@ -11,9 +11,9 @@ The reference network definitions (``unet.py``, ``attention.py``, ``layer_norm.p
 
 Both are replaced by the minimal stand-ins below (SURVEY.md section 8c lists the exact
 requirements).  No reference source is copied: the modules are imported from where they lie
-(``$B200SD_REFERENCE``, ``baseline/_ref`` or ``/root/reference``).  On the GPU box the
-reference tree does not exist; callers must check :func:`available` and fall back to
-``oracle.restated`` + the committed golden fixtures.
+(``$B200SD_REFERENCE`` or ``baseline/_ref``).  Only the golden-fixture generators under
+``tests/golden/`` need the reference tree; the tests compare against the fixtures they wrote and
+``oracle.restated``.
 """
 from __future__ import annotations
 
@@ -29,7 +29,6 @@ _REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 _CANDIDATES = [
     os.environ.get("B200SD_REFERENCE", ""),
     os.path.join(_REPO, "baseline", "_ref"),
-    "/root/reference",
 ]
 
 

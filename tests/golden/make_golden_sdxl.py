@@ -1,8 +1,8 @@
 """Golden fixture for BASELINE configs[3]: SDXL-base UNet (UNet2DConditionModelXL, 2.57 B parameters) at 768x768
 (96x96 latents), produced by the UNMODIFIED reference modules on the CPU in fp32 (about 10 GB of RAM, a few
-minutes).  Build container only:
+minutes):
 
-    python tests/golden/make_golden_sdxl.py
+    B200SD_REFERENCE=<reference checkout> python tests/golden/make_golden_sdxl.py
 
 Weights are regenerated from the seed on the test side (see make_golden.py); stored: the inputs that are not
 seed-derived, the reference output and a weight fingerprint.

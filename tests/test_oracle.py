@@ -1,5 +1,7 @@
-"""CPU tests that pin the oracle (oracle/restated.py) against (a) the golden vectors produced by the
-unmodified reference modules and (b) the reference modules themselves when the tree is present."""
+"""CPU tests that pin the oracle (oracle/restated.py) and the engine's parameter schemas against the golden
+fixtures produced by the unmodified reference modules (tests/golden/make_golden*.py)."""
+import gzip
+import json
 import os
 
 import numpy as np
@@ -7,7 +9,7 @@ import pytest
 import torch
 
 from b200sd import config
-from oracle import ref_unet, restated as R
+from oracle import restated as R
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 sys_path_inserted = True
@@ -15,6 +17,12 @@ sys_path_inserted = True
 
 def _load(name):
     return np.load(os.path.join(GOLD, name))
+
+
+def _reference_schema(name):
+    """{parameter name: shape} of the reference module built from config.<name>."""
+    with gzip.open(os.path.join(GOLD, "param_schemas.json.gz"), "rt") as f:
+        return {k: tuple(v) for k, v in json.load(f)[name].items()}
 
 
 def _fingerprint(sd):
@@ -69,52 +77,63 @@ def test_restated_xl_and_controlnet_match_reference_golden():
         assert np.abs(o.numpy() - gold[f"residual_{i}"]).max() < 2e-5, i
 
 
-@pytest.mark.skipif(not ref_unet.available(), reason="reference tree not present on this box")
 def test_controlnet_schema_matches_reference_modules():
-    for cfg in (config.TINY_CONTROLNET, config.SD21_CONTROLNET):
-        with torch.device("meta"):
-            m = ref_unet.build_controlnet(cfg)
-        ref_shapes = {k: tuple(v.shape) for k, v in m.state_dict().items()}
-        assert ref_shapes == {k: tuple(v) for k, v in config.controlnet_param_shapes(cfg).items()}
+    for name in ("TINY_CONTROLNET", "SD21_CONTROLNET"):
+        ref_shapes = _reference_schema(name)
+        mine = {k: tuple(v) for k, v in config.controlnet_param_shapes(getattr(config, name)).items()}
+        assert ref_shapes == mine, (name, set(ref_shapes.items()) ^ set(mine.items()))
+
+
+def _block_inputs(seed):
+    """The operands make_golden.block_inputs drew for blocks.npz."""
+    g = torch.Generator().manual_seed(seed)
+    q = torch.randn(2, 128, 1, 200, generator=g)
+    k = torch.randn(2, 128, 1, 77, generator=g)
+    v = torch.randn(2, 128, 1, 77, generator=g)
+    w = torch.randn(128, generator=g)
+    b = torch.randn(128, generator=g)
+    mask = torch.zeros(2, 77, 1, 1)
+    mask[:, 50:] = -1e4
+    return q, k, v, mask, w, b
 
 
 def test_restated_blocks_match_reference_golden():
     g = _load("blocks.npz")
-    q, k, v = (torch.from_numpy(g[n]) for n in "qkv")
+    q, k, v, mask, w, b = _block_inputs(int(g["input_seed"]))
+    fp = np.array([float(t.double().sum()) for t in (q, k, v, w, b)])
+    assert np.allclose(fp, g["input_fingerprint"], rtol=1e-6), "input generator drifted"
     ref = R.attention(q, k, v, 2, 64).numpy()
     for nm in ("original", "split_einsum", "split_einsum_v2"):
         assert np.abs(ref - g[f"attn_{nm}"]).max() < 2e-6, nm
-    masked = R.attention(q, k, v, 2, 64, mask=torch.from_numpy(g["mask"])).numpy()
+    masked = R.attention(q, k, v, 2, 64, mask=mask).numpy()
     assert np.abs(masked - g["attn_split_einsum_masked"]).max() < 2e-6
     # LayerNormANE is (x_hat + b) * w; the oracle/engine convention is x_hat * w + b' with b' = b * w
-    w, b = torch.from_numpy(g["ln_weight"]), torch.from_numpy(g["ln_bias"])
     ln = R.layer_norm_channels(q, w, b * w).numpy()
     assert np.abs(ln - g["ln_out"]).max() < 2e-5
     temb = R.timestep_embedding(torch.tensor([981.0, 1.0, 500.0]), 320).numpy()
     assert np.abs(temb - g["temb"]).max() < 1e-6
 
 
-@pytest.mark.skipif(not ref_unet.available(), reason="reference tree not present on this box")
 def test_param_schema_matches_reference_modules():
-    for cfg, xl in ((config.TINY_UNET, False), (config.SD21_BASE_UNET, False), (config.SDXL_BASE_UNET, True)):
-        with torch.device("meta"):
-            m = ref_unet.build_unet(cfg, None, xl=xl)
-        ref_shapes = {k: tuple(v.shape) for k, v in m.state_dict().items()}
-        mine = {k: tuple(v) for k, v in config.unet_param_shapes(cfg).items()}
-        assert ref_shapes == mine
+    for name in ("TINY_UNET", "SD21_BASE_UNET", "SDXL_BASE_UNET"):
+        ref_shapes = _reference_schema(name)
+        mine = {k: tuple(v) for k, v in config.unet_param_shapes(getattr(config, name)).items()}
+        assert ref_shapes == mine, (name, set(ref_shapes.items()) ^ set(mine.items()))
 
 
-@pytest.mark.skipif(not ref_unet.available(), reason="reference tree not present on this box")
 def test_restated_matches_live_reference_tiny_all_impls():
+    """Tiny UNet with a different timestep per batch row against the reference's output under each of its three
+    attention implementations (unet_tiny_timesteps.npz)."""
+    gold = _load("unet_tiny_timesteps.npz")
     cfg = config.TINY_UNET
-    sd = config.random_state_dict(config.unet_param_shapes(cfg), seed=7)
-    x, c = _inputs(cfg, 8)
-    t = torch.tensor([501.0, 21.0])
+    sd = config.random_state_dict(config.unet_param_shapes(cfg), seed=int(gold["weight_seed"]))
+    assert np.allclose(_fingerprint(sd), gold["fingerprint"], rtol=1e-6), "weight generator drifted"
+    x, c = _inputs(cfg, int(gold["input_seed"]))
+    t = torch.from_numpy(gold["timesteps"])
     with torch.no_grad():
-        y = R.unet_forward(sd, cfg, x, t, c)
-        for impl in ("ORIGINAL", "SPLIT_EINSUM", "SPLIT_EINSUM_V2"):
-            m = ref_unet.build_unet(cfg, sd, impl=impl)
-            assert (m(x, t, c)[0] - y).abs().max() < 2e-5, impl
+        y = R.unet_forward(sd, cfg, x, t, c).numpy()
+    for impl in ("ORIGINAL", "SPLIT_EINSUM", "SPLIT_EINSUM_V2"):
+        assert np.abs(y - gold[f"noise_pred_{impl}"]).max() < 2e-5, impl
 
 
 def test_compute_psnr_definition():

@@ -1,15 +1,14 @@
-"""BPE tokenizer: algorithm on a tiny hand-made vocabulary (runs anywhere) and the reference's known-answer ids
-(StableDiffusionTests.swift:43-48) with the CLIP vocabulary / merges that ship inside the reference tree (build
-container only: the files are data of the reference and are not copied into this repository)."""
+"""BPE tokenizer: algorithm on a tiny hand-made vocabulary and the reference's known-answer ids
+(StableDiffusionTests.swift:43-48) with the part of the reference's CLIP vocabulary / merges that those prompts use
+(tests/golden/make_golden_tokenizer.py)."""
 import json
 import os
 
 import numpy as np
-import pytest
 
 from b200sd.tokenizer import BPETokenizer
 
-RES = "/root/reference/swift/StableDiffusionTests/Resources"
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def test_bpe_merges_by_rank_and_pads(tmp_path):
@@ -33,9 +32,9 @@ def test_bpe_merges_by_rank_and_pads(tmp_path):
     assert padded.input_ids("low") == [0, 2, 1, 7, 7, 7]
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(RES, "vocab.json")), reason="reference resources not present")
 def test_reference_known_answer_ids():
-    tok = BPETokenizer.from_files(os.path.join(RES, "merges.txt"), os.path.join(RES, "vocab.json"))
+    tok = BPETokenizer.from_files(os.path.join(GOLD, "clip_bpe_merges_subset.txt"),
+                                  os.path.join(GOLD, "clip_bpe_vocab_subset.json"))
     cases = {
         "a photo of an astronaut riding a horse on mars":
             [49406, 320, 1125, 539, 550, 18376, 6765, 320, 4558, 525, 7496, 49407],
