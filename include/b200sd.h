@@ -261,6 +261,30 @@ int b200sd_cfg_scheduler_step(const float* noise_pred, float* latents, float* hi
                               int32_t n, int32_t c, int32_t h, int32_t w,
                               const b200sd_step_coeffs* coeffs /* host */, void* stream);
 
+/* ---- sampler step: the CFG + scheduler step above, extended for the sigma-space and stochastic samplers ----
+ * (EulerDiscrete, EulerAncestralDiscrete, LMSDiscrete, DDIM with eta > 0; pipeline.py:504-508 scale_model_input)
+ *     x_prev  = <the linear update of b200sd_step_coeffs> + noise_scale * z
+ *     unet_in = fp16(in_scale * x_prev)     (in_scale: the NEXT step's c_in = 1 / sqrt(sigma^2 + 1))
+ * z is a standard normal from Philox-4x32-10 keyed by rng_key[0..1] (device memory, so a new seed needs no graph
+ * recapture), counter (noise_draw + b, 0, element index within image b, 0), Box-Muller on the first two words in
+ * double precision rounded once to fp32: the stream of the Swift pipeline's nvidiaRNG (rng.py NvRandomSource), so
+ * draw d of this kernel equals the d-th normal_array() call of a NvRandomSource with the same seed.
+ * noise_pred == NULL selects the input-only mode: unet_in = fp16(in_scale * latents), nothing else is read or written
+ * (the first UNet input of a loop).  With in_scale == 1 and noise_scale == 0 the arithmetic is that of
+ * b200sd_cfg_scheduler_step, bit for bit.  rng_key may be NULL when noise_scale == 0. */
+typedef struct {
+    b200sd_step_coeffs step;
+    float in_scale;          /* multiplies the value written to unet_in */
+    float noise_scale;       /* 0: no noise term */
+    uint32_t noise_draw;     /* Philox counter word 0 of image 0; image b uses noise_draw + b */
+} b200sd_sampler_coeffs;
+
+int b200sd_sampler_step(const float* noise_pred /* or NULL: input-only mode */, float* latents,
+                        float* hist /* [4][numel] */, float* denoised /* x0 out or NULL */, void* unet_in,
+                        int32_t c_pad, int32_t n, int32_t c, int32_t h, int32_t w,
+                        const b200sd_sampler_coeffs* coeffs /* host */, const uint32_t* rng_key /* device, 2 words */,
+                        void* stream);
+
 /* VAE decoder input: out = post_quant_conv(z * inv_scale) as NHWC fp16 padded to c_pad channels
  * (pipeline.py:313-316 `z / 0.18215`; torch2coreml.py:590-594 post_quant_conv); z fp32 NCHW, c <= 8,
  * w fp32 [c, c], b fp32 [c]. */

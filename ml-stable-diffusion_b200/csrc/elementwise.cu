@@ -211,15 +211,51 @@ __global__ void timestep_embedding_kernel(const float* __restrict__ t, float* __
 }
 
 // ---- fused CFG + scheduler step ------------------------------------------------------------------
-// One thread per latent element (n*c*h*w, NCHW fp32).  See include/b200sd.h for the algebra.
+// Philox-4x32-10 normal (rng.py NvRandomSource, the Swift pipeline's nvidiaRNG): counter (draw, 0, idx, 0), Box-Muller on
+// the first two output words in double precision, rounded once to fp32.  The explicit _rn intrinsics keep the compiler
+// from contracting the uniform maps into FMAs, which the host twin does not do.
+__device__ __forceinline__ float philox_normal(uint32_t k0, uint32_t k1, uint32_t draw, uint32_t idx) {
+    uint32_t c0 = draw, c1 = 0u, c2 = idx, c3 = 0u;
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint64_t v1 = static_cast<uint64_t>(c0) * 0xD2511F53ull;
+        const uint64_t v2 = static_cast<uint64_t>(c2) * 0xCD9E8D57ull;
+        c0 = static_cast<uint32_t>(v2 >> 32) ^ c1 ^ k0;
+        c1 = static_cast<uint32_t>(v2);
+        c2 = static_cast<uint32_t>(v1 >> 32) ^ c3 ^ k1;
+        c3 = static_cast<uint32_t>(v1);
+        k0 += 0x9E3779B9u;
+        k1 += 0xBB67AE85u;
+    }
+    const double u = __dadd_rn(__dmul_rn(static_cast<double>(c0), 1.0 / 4294967296.0), 1.0 / 8589934592.0);
+    const double v = __dadd_rn(__dmul_rn(static_cast<double>(c1), 3.141592653589793 / 2147483648.0),
+                               3.141592653589793 / 4294967296.0);
+    return static_cast<float>(__dmul_rn(sqrt(-2.0 * log(u)), sin(v)));
+}
+
+// One thread per latent element (n*c*h*w, NCHW fp32).  See include/b200sd.h for the algebra.  kExt = false is the
+// plain CFG + scheduler step (b200sd_cfg_scheduler_step); kExt = true adds the sampler terms (input scale, noise,
+// input-only mode) of b200sd_sampler_step.
+template <bool kExt>
 __global__ void cfg_step_kernel(const float* __restrict__ noise_pred, float* __restrict__ latents,
                                 float* __restrict__ hist, float* __restrict__ denoised, __half* __restrict__ unet_in,
-                                int c_pad, int n, int c, int hw, b200sd_step_coeffs k) {
+                                int c_pad, int n, int c, int hw, b200sd_sampler_coeffs sk,
+                                const uint32_t* __restrict__ rng_key) {
     pdl_trigger();  // no TMEM / large shared memory here: dependents may start their prologue at once
     pdl_wait();
+    const b200sd_step_coeffs& k = sk.step;
     const int numel = n * c * hw;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= numel) return;
+    if (kExt && !noise_pred) {  // input-only mode: the first UNet input of a loop
+        const int p = i % hw;
+        const int ch = (i / hw) % c;
+        const int b = i / (hw * c);
+        const __half hv = __float2half_rn(sk.in_scale * latents[i]);
+        unet_in[(static_cast<size_t>(b) * hw + p) * c_pad + ch] = hv;
+        unet_in[(static_cast<size_t>(n + b) * hw + p) * c_pad + ch] = hv;
+        return;
+    }
     int ni = i;  // index of this element inside one CFG half of noise_pred
     if (k.noise_pred_nhwc) {  // the UNet's conv_out output as it leaves the epilogue: [2n, h*w, c]
         const int p = i % hw;
@@ -241,6 +277,13 @@ __global__ void cfg_step_kernel(const float* __restrict__ noise_pred, float* __r
             x0 += k.x0_ch[j] * hv;
         }
     }
+    if (kExt && sk.noise_scale != 0.f) {  // no "+ 0 * z": that would turn a -0 into +0
+        const int per = c * hw;
+        const int b = i / per;
+        const float z = philox_normal(rng_key[0], rng_key[1], sk.noise_draw + static_cast<uint32_t>(b),
+                                      static_cast<uint32_t>(i - b * per));
+        xp += sk.noise_scale * z;
+    }
     if (k.push_eps_slot >= 0) hist[static_cast<size_t>(k.push_eps_slot) * numel + i] = eps;
     if (k.push_x0_slot >= 0) hist[static_cast<size_t>(k.push_x0_slot) * numel + i] = x0;
     if (k.push_x_slot >= 0) hist[static_cast<size_t>(k.push_x_slot) * numel + i] = x;
@@ -251,7 +294,7 @@ __global__ void cfg_step_kernel(const float* __restrict__ noise_pred, float* __r
         const int p = i % hw;
         const int ch = (i / hw) % c;
         const int b = i / (hw * c);
-        const __half hv = __float2half_rn(xp);
+        const __half hv = __float2half_rn(kExt && sk.in_scale != 1.f ? sk.in_scale * xp : xp);
         unet_in[(static_cast<size_t>(b) * hw + p) * c_pad + ch] = hv;
         unet_in[(static_cast<size_t>(n + b) * hw + p) * c_pad + ch] = hv;
     }
@@ -440,24 +483,50 @@ extern "C" int b200sd_timestep_embedding(const float* timesteps, float* out, int
     return 0;
 }
 
+static int launch_step(const char* what, const float* noise_pred, float* latents, float* hist, float* denoised,
+                       void* unet_in, int32_t c_pad, int32_t n, int32_t c, int32_t h, int32_t w,
+                       const b200sd_sampler_coeffs& sk, const uint32_t* rng_key, bool ext, cudaStream_t stream) {
+    const b200sd_step_coeffs* coeffs = &sk.step;
+    if (noise_pred) {  // the input-only mode reads no history
+    B200SD_REQUIRE(coeffs->n_hist >= 0 && coeffs->n_hist <= 4 && (coeffs->n_hist == 0 || hist),
+                   "%s: bad history arguments", what);
+    B200SD_REQUIRE(coeffs->push_eps_slot < 4 && coeffs->push_x0_slot < 4 && coeffs->push_x_slot < 4 &&
+                       (hist || (coeffs->push_eps_slot < 0 && coeffs->push_x0_slot < 0 && coeffs->push_x_slot < 0)),
+                   "%s: bad history ring slot", what);
+    }
+    const int numel = n * c * h * w;
+    B200SD_CHECK_CUDA(launch_kernel(ext ? cfg_step_kernel<true> : cfg_step_kernel<false>, dim3((numel + 255) / 256),
+                                    dim3(256), 0, stream, noise_pred, latents, hist, denoised,
+                                    reinterpret_cast<__half*>(unet_in), c_pad, n, c, h * w, sk, rng_key));
+    B200SD_CHECK_CUDA(cudaGetLastError());
+    count_launch(1);
+    return 0;
+}
+
 extern "C" int b200sd_cfg_scheduler_step(const float* noise_pred, float* latents, float* hist, float* denoised,
                                          void* unet_in, int32_t c_pad, int32_t n, int32_t c, int32_t h, int32_t w,
                                          const b200sd_step_coeffs* coeffs, void* stream_) {
     if (!b200sd::launch_class_enabled(8)) return 0;  // bench.py's per-class timing graphs
-    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     B200SD_REQUIRE(noise_pred && latents && coeffs, "b200sd_cfg_scheduler_step: null pointer");
-    B200SD_REQUIRE(coeffs->n_hist >= 0 && coeffs->n_hist <= 4 && (coeffs->n_hist == 0 || hist),
-                   "b200sd_cfg_scheduler_step: bad history arguments");
-    B200SD_REQUIRE(coeffs->push_eps_slot < 4 && coeffs->push_x0_slot < 4 && coeffs->push_x_slot < 4 &&
-                       (hist || (coeffs->push_eps_slot < 0 && coeffs->push_x0_slot < 0 && coeffs->push_x_slot < 0)),
-                   "b200sd_cfg_scheduler_step: bad history ring slot");
-    const int numel = n * c * h * w;
-    B200SD_CHECK_CUDA(launch_kernel(cfg_step_kernel, dim3((numel + 255) / 256), dim3(256), 0, stream, noise_pred, latents, hist, denoised,
-                                                             reinterpret_cast<__half*>(unet_in), c_pad, n, c, h * w,
-                                                             *coeffs));
-    B200SD_CHECK_CUDA(cudaGetLastError());
-    count_launch(1);
-    return 0;
+    b200sd_sampler_coeffs sk{};
+    sk.step = *coeffs;
+    sk.in_scale = 1.f;
+    return launch_step("b200sd_cfg_scheduler_step", noise_pred, latents, hist, denoised, unet_in, c_pad, n, c, h, w, sk,
+                       nullptr, false, static_cast<cudaStream_t>(stream_));
+}
+
+extern "C" int b200sd_sampler_step(const float* noise_pred, float* latents, float* hist, float* denoised, void* unet_in,
+                                   int32_t c_pad, int32_t n, int32_t c, int32_t h, int32_t w,
+                                   const b200sd_sampler_coeffs* coeffs, const uint32_t* rng_key, void* stream_) {
+    if (!b200sd::launch_class_enabled(8)) return 0;  // bench.py's per-class timing graphs
+    B200SD_REQUIRE(latents && coeffs, "b200sd_sampler_step: null pointer");
+    B200SD_REQUIRE(noise_pred || (unet_in && c_pad >= c), "b200sd_sampler_step: the input-only mode needs unet_in");
+    B200SD_REQUIRE(coeffs->noise_scale == 0.f || !noise_pred || rng_key,
+                   "b200sd_sampler_step: noise_scale != 0 needs rng_key");
+    // with the sampler terms off this is the plain step kernel, so those samplers keep its arithmetic exactly
+    const bool ext = !noise_pred || coeffs->in_scale != 1.f || coeffs->noise_scale != 0.f;
+    return launch_step("b200sd_sampler_step", noise_pred, latents, hist, denoised, unet_in, c_pad, n, c, h, w, *coeffs,
+                       rng_key, ext, static_cast<cudaStream_t>(stream_));
 }
 
 extern "C" int b200sd_image_postprocess(const void* in, int32_t in_f32, int32_t c_pad, float* out_f32,

@@ -49,6 +49,11 @@ class StepCoeffs(C.Structure):
     ]
 
 
+class SamplerCoeffs(C.Structure):
+    """b200sd_sampler_coeffs: the step coefficients + input scale, noise scale and Philox draw index."""
+    _fields_ = [("step", StepCoeffs), ("in_scale", C.c_float), ("noise_scale", C.c_float), ("noise_draw", C.c_uint32)]
+
+
 _SIGNATURES = {
     "b200sd_last_error": (C.c_char_p, []),
     "b200sd_version": (C.c_int, []),
@@ -105,6 +110,8 @@ _SIGNATURES = {
     "b200sd_cfg_scheduler_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                             C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(StepCoeffs),
                                             C.c_void_p]),
+    "b200sd_sampler_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
+                                      C.c_int32, C.c_int32, C.c_int32, C.POINTER(SamplerCoeffs), C.c_void_p, C.c_void_p]),
     "b200sd_image_postprocess": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32,
                                            C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
 }
@@ -616,6 +623,21 @@ def cfg_scheduler_step(noise_pred, latents, coeffs: StepCoeffs, hist=None, denoi
     _check(load().b200sd_cfg_scheduler_step(_ptr(noise_pred), _ptr(latents), _ptr(hist), _ptr(denoised),
                                             _ptr(unet_in), c_pad, n, c, h, w, C.byref(coeffs), _stream()),
            "b200sd_cfg_scheduler_step")
+    return latents
+
+
+def sampler_step(noise_pred, latents, coeffs: SamplerCoeffs, hist=None, denoised=None, unet_in=None, rng_key=None):
+    """b200sd_sampler_step.  noise_pred None: input-only mode (unet_in = fp16(in_scale * latents)); rng_key: int32 CUDA
+    tensor of 2 words (the Philox key), needed when coeffs.noise_scale != 0."""
+    if noise_pred is not None:
+        _req(noise_pred, torch.float32, "sampler_step noise_pred")
+    _req(latents, torch.float32, "sampler_step latents")
+    if rng_key is not None and (rng_key.dtype != torch.int32 or not rng_key.is_cuda or rng_key.numel() < 2):
+        raise B200SDError("sampler_step: rng_key must be a CUDA int32 tensor of 2 words")
+    n, c, h, w = latents.shape
+    c_pad = 0 if unet_in is None else unet_in.shape[-1]
+    _check(load().b200sd_sampler_step(_ptr(noise_pred), _ptr(latents), _ptr(hist), _ptr(denoised), _ptr(unet_in), c_pad,
+                                      n, c, h, w, C.byref(coeffs), _ptr(rng_key), _stream()), "b200sd_sampler_step")
     return latents
 
 

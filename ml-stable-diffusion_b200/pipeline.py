@@ -107,6 +107,9 @@ class B200StableDiffusionPipeline:
         self._denoised = torch.zeros(n, c, h, w, dtype=torch.float32, device=dev)
         self._ctx = torch.zeros(2 * n, d_ctx, 1, unet.seq, dtype=torch.float16, device=dev)
         self._t = torch.zeros(2 * n, dtype=torch.float32, device=dev)
+        # Philox key of the samplers' per-step noise (b200sd_sampler_step): device memory, so a new seed is a copy, not a
+        # new loop graph
+        self._rng_key = torch.zeros(2, dtype=torch.int32, device=dev)
 
     # ---------------------------------------------------------------- factory
     @classmethod
@@ -154,6 +157,7 @@ class B200StableDiffusionPipeline:
                    tokenizer=tokenizer, vae_encoder=venc, force_zeros_for_empty_prompt=unet.engine.xl)
 
     _SCHEDULER_CLASS = {"PNDMScheduler": "PNDM", "DDIMScheduler": "DDIM", "DPMSolverMultistepScheduler": "DPMSolverMultistep"}
+    _SIGMA_SCHEDULERS = ("EulerDiscrete", "EulerAncestralDiscrete", "LMSDiscrete")
 
     @classmethod
     def from_pretrained(cls, model_dir, images_per_call=1, device="cuda", height=None, width=None,
@@ -213,9 +217,17 @@ class B200StableDiffusionPipeline:
         enc1, tok1 = text_pair("text_encoder", "tokenizer")
         enc2, tok2 = text_pair("text_encoder_2", "tokenizer_2")
         sched = scheduler_override
+        sched_cfg_path = os.path.join(model_dir, "scheduler", "scheduler_config.json")
+        sched_cfg = {}
+        if sched is None or os.path.exists(sched_cfg_path):  # without an override the config must exist
+            with open(sched_cfg_path) as fh:
+                sched_cfg = json.load(fh)
+        sched_kwargs = None
+        if sched in cls._SIGMA_SCHEDULERS:
+            # what the reference's from_config carries over to these classes (pipeline.py:816-821)
+            sched_kwargs = {k: sched_cfg[k] for k in ("timestep_spacing", "steps_offset") if k in sched_cfg}
         if sched is None:
-            with open(os.path.join(model_dir, "scheduler", "scheduler_config.json")) as fh:
-                name = json.load(fh).get("_class_name", "PNDMScheduler")
+            name = sched_cfg.get("_class_name", "PNDMScheduler")
             if name not in cls._SCHEDULER_CLASS:
                 raise ValueError(f"scheduler {name} of the checkpoint is not implemented; pass scheduler_override "
                                  f"(one of {sorted(S.SCHEDULER_MAP)})")
@@ -238,7 +250,7 @@ class B200StableDiffusionPipeline:
             force_zeros_for_empty_prompt = xl   # the reference's CLI sets it for SDXL only (pipeline.py:744-755)
         return cls(unet, vae, scheduler=sched, text_encoder=enc1, tokenizer=tok1, text_encoder_2=enc2, tokenizer_2=tok2,
                    xl=xl, controlnet=nets, vae_encoder=venc, force_zeros_for_empty_prompt=force_zeros_for_empty_prompt,
-                   unet_refiner=refiner)
+                   unet_refiner=refiner, scheduler_kwargs=sched_kwargs)
 
     # ---------------------------------------------------------------- reference-named helpers
     def check_inputs(self, prompt, height, width, callback_steps):
@@ -386,7 +398,31 @@ class B200StableDiffusionPipeline:
                                                                     st.push_x0_slot, st.push_x_slot)
         return k
 
-    def _loop_on_static_buffers(self, plan, guidance_scale, ts_rows, use_controlnet=False, refiner_start_step=None):
+    def _sampler_coeffs(self, st, guidance_scale, k=None):
+        """b200sd_sampler_coeffs of a step: the linear update + input scale, noise scale and this step's Philox draws."""
+        k = k or L.SamplerCoeffs()
+        self._coeffs(st, guidance_scale, k.step)
+        k.in_scale, k.noise_scale = st.in_scale, st.noise_scale
+        k.noise_draw = (self.images_per_call * st.noise_draw) & 0xFFFFFFFF
+        return k
+
+    def _make_scheduler(self, num_inference_steps, eta=0.0):
+        kw = dict(self.scheduler_kwargs)
+        if eta:  # like the reference (pipeline.py:384-396), eta reaches DDIM only and is ignored by the other schedulers
+            if self.scheduler_name == "DDIM":
+                kw["eta"] = float(eta)
+        return S.make_scheduler(self.scheduler_name, num_inference_steps, **kw)
+
+    def _set_noise_key(self, seed):
+        """The Philox key of the per-step noise: ``seed``, or with ``seed=None`` a draw from the global numpy stream,
+        taken after every other draw of the call."""
+        if seed is None:
+            seed = int(np.random.randint(0, 2 ** 32, dtype=np.uint64))
+        key = np.array([int(seed) & 0xFFFFFFFF, 0], dtype=np.uint32).view(np.int32)
+        self._rng_key.copy_(torch.from_numpy(key))
+
+    def _loop_on_static_buffers(self, plan, guidance_scale, ts_rows, use_controlnet=False, refiner_start_step=None,
+                                in_scale0=1.0):
         """The whole N-step loop on static device buffers (no host-side tensor arguments): what the loop graph
         captures.  Prologue, once per prompt: cross-attention K/V of all blocks from the text states, the
         time-embedding biases of all ResNet blocks for ALL timesteps (`ts_rows`: each step's timestep repeated per
@@ -409,17 +445,21 @@ class B200StableDiffusionPipeline:
         first = models[0]
         L.nchw_to_nhwc(self._latents, c_pad=first.engine.in_pad, out=first._x_nhwc[:n])
         L.nchw_to_nhwc(self._latents, c_pad=first.engine.in_pad, out=first._x_nhwc[n:])
+        if in_scale0 != 1.0:  # sigma-space samplers: the UNet sees c_in(sigma_0) * x (pipeline.py:504-508)
+            k0 = L.SamplerCoeffs()
+            k0.in_scale = in_scale0
+            L.sampler_step(None, self._latents, k0, unet_in=first._x_nhwc)
         if use_controlnet:
             self.prepare_controlnets(ts_rows)
         for i, st in enumerate(plan):
             u = models[i]
             table, lo = tables[id(u)]
             u._run_core(table[i - lo], self.controlnet_residuals(i) if use_controlnet else None)
-            k = self._coeffs(st, guidance_scale)
-            k.noise_pred_nhwc = 1
+            k = self._sampler_coeffs(st, guidance_scale)
+            k.step.noise_pred_nhwc = 1
             nxt = models[i + 1] if i + 1 < len(plan) else u
-            L.cfg_scheduler_step(u._out_nhwc, self._latents, k, hist=self._hist, denoised=self._denoised,
-                                 unet_in=nxt._x_nhwc)
+            L.sampler_step(u._out_nhwc, self._latents, k, hist=self._hist, denoised=self._denoised,
+                           unet_in=nxt._x_nhwc, rng_key=self._rng_key)
 
     def set_control_conditions(self, controlnet_cond):
         """Copy the conditioning images (each (2B, 3, H, W)) into the ControlNets' static input buffers."""
@@ -448,7 +488,7 @@ class B200StableDiffusionPipeline:
         return torch.tensor([float(st.timestep) for st in plan for _ in range(self.unet.batch)], dtype=torch.float32,
                             device=self.device)
 
-    def _loop_graph_for(self, key, plan, guidance_scale, use_controlnet=False, refiner_start_step=None):
+    def _loop_graph_for(self, key, plan, guidance_scale, use_controlnet=False, refiner_start_step=None, in_scale0=1.0):
         g = self._loop_graphs.get(key)
         if g is None:
             keep = self._latents.clone()
@@ -456,15 +496,17 @@ class B200StableDiffusionPipeline:
             s = torch.cuda.Stream(device=self.device)  # eager warm-up off the capture: workspaces, weight tiling
             s.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(s):
-                self._loop_on_static_buffers(plan[:1], guidance_scale, ts_rows[: self.unet.batch], use_controlnet)
+                self._loop_on_static_buffers(plan[:1], guidance_scale, ts_rows[: self.unet.batch], use_controlnet,
+                                             in_scale0=in_scale0)
                 if refiner_start_step is not None and refiner_start_step < len(plan):  # warm the refiner's kernels too
-                    self._loop_on_static_buffers(plan[-1:], guidance_scale, ts_rows[-self.unet.batch:], use_controlnet, 0)
+                    self._loop_on_static_buffers(plan[-1:], guidance_scale, ts_rows[-self.unet.batch:], use_controlnet, 0,
+                                                 in_scale0=in_scale0)
             torch.cuda.current_stream().wait_stream(s)
             torch.cuda.synchronize()
             self._latents.copy_(keep)
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
-                self._loop_on_static_buffers(plan, guidance_scale, ts_rows, use_controlnet, refiner_start_step)
+                self._loop_on_static_buffers(plan, guidance_scale, ts_rows, use_controlnet, refiner_start_step, in_scale0)
             g._b200sd_keep = ts_rows
             self._latents.copy_(keep)  # capture does not execute, but keep the contract obvious
             if len(self._loop_graphs) >= 4:
@@ -474,14 +516,20 @@ class B200StableDiffusionPipeline:
 
     def denoise(self, text_embeddings, latents, num_inference_steps, guidance_scale, callback=None,
                 callback_steps=1, time_ids=None, text_embeds=None, return_denoised=False, record=None,
-                controlnet_cond=None, start_step=0, refiner=None, refiner_start=0.8):
+                controlnet_cond=None, start_step=0, refiner=None, refiner_start=0.8, eta=0.0, seed=None):
         """Runs the N-step loop (from ``start_step``: image-to-image) entirely on the device.  ``text_embeddings`` (2B, D, 1, S) and ``latents``
         (B, C, h, w) may be numpy (copied once, before the loop) or CUDA tensors.  ``record`` (a list) receives
         (timestep, noise_pred, latents_after_step) clones per step -- a debugging / testing aid.  Without
         callback / record / ControlNet the whole loop replays as ONE CUDA graph (SURVEY 8f N1): the scheduler
-        history lives on the device and no host synchronisation happens between the first and the last step."""
-        sched = S.make_scheduler(self.scheduler_name, num_inference_steps, **self.scheduler_kwargs)
+        history lives on the device and no host synchronisation happens between the first and the last step.
+        ``latents`` are in the scheduler's own space (already multiplied by ``init_noise_sigma``, ``__call__`` does
+        that).  ``eta``: DDIM's noise weight.  ``seed``: the Philox key of the per-step noise of Euler-ancestral and
+        DDIM eta > 0 (``None``: drawn from the global numpy stream); it is not part of the loop graph."""
+        sched = self._make_scheduler(num_inference_steps, eta)
         plan = list(sched.plan(start=start_step)) if start_step else list(sched.plan())
+        in_scale0 = sched.first_in_scale(start_step)
+        if sched.uses_noise:
+            self._set_noise_key(seed)
         n = self.images_per_call
         self._ctx.copy_(torch.as_tensor(text_embeddings), non_blocking=True)
         self._latents.copy_(torch.as_tensor(latents), non_blocking=True)
@@ -510,24 +558,30 @@ class B200StableDiffusionPipeline:
                 r._text_embeds.copy_(torch.as_tensor(refiner["text_embeds"]))
                 rstep = int(np.float32(len(plan)) * np.float32(refiner_start))  # Int(Float(timeSteps.count) * refinerStart)
             key = (self.scheduler_name, int(num_inference_steps), float(guidance_scale), int(start_step),
-                   bool(controlnet_cond), tuple(sorted(self.scheduler_kwargs.items())), rstep)
-            self._loop_graph_for(key, plan, guidance_scale, bool(controlnet_cond), rstep).replay()
+                   bool(controlnet_cond), tuple(sorted(self.scheduler_kwargs.items())), rstep, float(eta))
+            self._loop_graph_for(key, plan, guidance_scale, bool(controlnet_cond), rstep, in_scale0).replay()
             return self._denoised if return_denoised else self._latents
         if refiner is not None:
             raise ValueError("the refiner hand-off runs in the device loop only (no callback / record)")
         self._hist.zero_()
-        k = L.StepCoeffs()
+        k = L.SamplerCoeffs()
+        scale = in_scale0
         for i, st in enumerate(plan):
             self._t.fill_(float(st.timestep))
             sample = torch.cat([self._latents, self._latents], 0)  # pipeline.py:502
+            if scale != 1.0:
+                # scale_model_input (pipeline.py:504-508): the fp32 product the step kernel writes to the loop graph's
+                # UNet input, rounded to fp16 by the same conversion, so both paths feed the UNet the same bits
+                sample.mul_(float(np.float32(scale)))
             residuals = None
             if controlnet_cond:  # pipeline.py:515-529
                 residuals = self.run_controlnet(sample, self._t, self._ctx, controlnet_cond)
             noise_pred = self.unet.forward_device(sample, self._t, self._ctx, time_ids, text_embeds, residuals)
-            self._coeffs(st, guidance_scale, k)
+            self._sampler_coeffs(st, guidance_scale, k)
+            scale = st.in_scale
             if record is not None:
                 eps_copy = noise_pred.clone()
-            L.cfg_scheduler_step(noise_pred, self._latents, k, hist=self._hist, denoised=self._denoised)
+            L.sampler_step(noise_pred, self._latents, k, hist=self._hist, denoised=self._denoised, rng_key=self._rng_key)
             if record is not None:
                 record.append((st.timestep, eps_copy, self._latents.clone()))
             if callback is not None and i % callback_steps == 0:
@@ -558,8 +612,8 @@ class B200StableDiffusionPipeline:
         width = width or self.width
         if (height, width) != (self.height, self.width):
             raise ValueError(f"this pipeline instance was built for {self.height}x{self.width} images")
-        if eta != 0.0:
-            raise ValueError("only eta = 0 (deterministic DDIM) is implemented")
+        if eta < 0:
+            raise ValueError(f"eta must be >= 0, got {eta}")
         if controlnet_cond and not self.controlnet:
             raise ValueError("Conditions for controlnet are given but the pipeline has no controlnet modules")
         prompts = [prompt] if isinstance(prompt, str) else list(prompt)
@@ -588,11 +642,13 @@ class B200StableDiffusionPipeline:
             if text_embeds is None:
                 text_embeds = torch.zeros(2 * self.images_per_call, 1280, device=self.device)
         lat = self.prepare_latents(len(prompts), self.unet.in_channels, height, width, latents, seed=seed, rng=rng)
+        sched = self._make_scheduler(num_inference_steps, eta)
         start_step = 0
+        if starting_image is None and sched.init_noise_sigma != 1.0:
+            lat = lat * np.float32(sched.init_noise_sigma)  # pipeline.py:344 (sigma-space samplers)
         if starting_image is not None:
             if self.vae_encoder is None:
                 raise ValueError("a starting image was provided but the pipeline has no vae_encoder")
-            sched = S.make_scheduler(self.scheduler_name, num_inference_steps, **self.scheduler_kwargs)
             start_step = sched.start_step(strength)
             if start_step >= num_inference_steps:
                 raise ValueError(f"strength {strength} leaves no denoising steps")
@@ -621,7 +677,7 @@ class B200StableDiffusionPipeline:
                        "time_ids": torch.tensor(rows, dtype=torch.float32)}
         final = self.denoise(text_embeddings, lat, num_inference_steps, guidance_scale, callback, callback_steps,
                              time_ids, text_embeds, controlnet_cond=controlnet_cond or None, start_step=start_step,
-                             refiner=refiner, refiner_start=refiner_start)
+                             refiner=refiner, refiner_start=refiner_start, eta=eta, seed=seed)
         image = self.decode_latents(final).cpu().numpy()  # single device->host copy of the result
         has_nsfw = None  # the safety checker is out of scope (SURVEY section 2, row 19)
         if output_type == "pil":

@@ -13,6 +13,14 @@ scheduler only produces, per step, the scalars of
 plus which history slots to overwrite; ``b200sd_cfg_scheduler_step`` applies them on the device
 (one launch, also does classifier-free guidance and writes the next UNet input), so the denoising
 loop never synchronises with the host.  Coefficients are computed in float64 and rounded once.
+
+The sigma-space samplers of diffusers 0.30.2 (EulerDiscrete, EulerAncestralDiscrete, LMSDiscrete), which the
+reference's Python pipeline offers (``pipeline.py:592-604``), and DDIM with eta > 0 add three per-step terms that the
+same kernel (``b200sd_sampler_step``) applies: ``in_scale``, the NEXT step's ``c_in = 1 / sqrt(sigma^2 + 1)``
+(``scale_model_input``, pipeline.py:504-508) on the value written as the next UNet input; ``noise_scale`` times a
+Philox normal drawn on the device (Euler-ancestral ``sigma_up``, DDIM's ``std_dev_t``); and ``noise_draw``, which block
+of that Philox stream the step uses (image ``b`` of ``n`` draws ``n * noise_draw + b``; draws ``0 .. n-1`` are the
+initial latents of ``rng="nvidia"``).
 """
 from __future__ import annotations
 
@@ -25,8 +33,8 @@ import numpy as np
 
 @dataclasses.dataclass
 class StepPlan:
-    """One denoising step: UNet timestep + the linear-update coefficients."""
-    timestep: int
+    """One denoising step: UNet timestep + the linear-update coefficients (+ the sampler terms, see the module doc)."""
+    timestep: float
     cx: float
     ce: float
     ch: List[float]
@@ -37,6 +45,9 @@ class StepPlan:
     push_eps_slot: int = -1
     push_x0_slot: int = -1
     push_x_slot: int = -1
+    in_scale: float = 1.0
+    noise_scale: float = 0.0
+    noise_draw: int = 0
 
 
 def alphas_cumprod(beta_start=0.00085, beta_end=0.012, n=1000, schedule="scaled_linear"):
@@ -65,6 +76,14 @@ class _Base:
     def scale_model_input(self, x, t):  # identity for DDIM / PNDM / DPM (pipeline.py:504)
         return x
 
+    def first_in_scale(self, start: int = 0) -> float:
+        """Scale of the first UNet input of a loop that starts at ``start`` (the later ones are ``StepPlan.in_scale``)."""
+        return 1.0
+
+    @property
+    def uses_noise(self) -> bool:
+        return False
+
     @property
     def timesteps(self):
         return [p.timestep for p in self.plan()]
@@ -91,25 +110,39 @@ class _Base:
 
 
 class DDIMScheduler(_Base):
-    """eta = 0, epsilon prediction, 'leading' spacing, steps_offset 1, set_alpha_to_one False."""
+    """Epsilon prediction, 'leading' spacing, steps_offset 1, set_alpha_to_one False.  ``eta`` > 0 adds
+    ``std_dev_t = eta * sqrt((1 - a_p) / (1 - a_t) * (1 - a_t / a_p))`` times fresh noise and takes ``std_dev_t^2`` out
+    of the direction term (diffusers 0.30.2 ``DDIMScheduler.step``); eta = 0 is the deterministic update."""
 
-    def __init__(self, num_inference_steps, steps_offset=1, **kw):
+    def __init__(self, num_inference_steps, steps_offset=1, eta=0.0, **kw):
         super().__init__(num_inference_steps, **kw)
         self.steps_offset = steps_offset
+        self.eta = float(eta)
+        if self.eta < 0:
+            raise ValueError(f"eta must be >= 0, got {eta}")
+
+    @property
+    def uses_noise(self):
+        return self.eta != 0.0
 
     def plan(self, start=0):
         ratio = self.n_train // self.n
         ts = [int(round(i * ratio)) + self.steps_offset for i in range(self.n)][::-1]
         out = []
-        for t in ts[start:]:
+        for j, t in enumerate(ts[start:]):
             tp = t - ratio
             a_t = self.abar[t]
             a_p = self.abar[tp] if tp >= 0 else self.abar[0]
             x0_cx = 1.0 / math.sqrt(a_t)
             x0_ce = -math.sqrt(1 - a_t) / math.sqrt(a_t)
             cx = math.sqrt(a_p) * x0_cx
-            ce = math.sqrt(a_p) * x0_ce + math.sqrt(1 - a_p)
-            out.append(StepPlan(t, cx, ce, [0.0] * 4, x0_cx, x0_ce, [0.0] * 4))
+            if self.eta == 0.0:
+                ce = math.sqrt(a_p) * x0_ce + math.sqrt(1 - a_p)
+                out.append(StepPlan(t, cx, ce, [0.0] * 4, x0_cx, x0_ce, [0.0] * 4))
+                continue
+            std = self.eta * math.sqrt((1 - a_p) / (1 - a_t) * (1 - a_t / a_p))
+            ce = math.sqrt(a_p) * x0_ce + math.sqrt(max(1 - a_p - std * std, 0.0))
+            out.append(StepPlan(t, cx, ce, [0.0] * 4, x0_cx, x0_ce, [0.0] * 4, noise_scale=std, noise_draw=1 + j))
         return out
 
 
@@ -246,9 +279,133 @@ class PNDMScheduler(_Base):
         return out
 
 
+class _SigmaBase(_Base):
+    """Shared schedule of the sigma-space samplers (diffusers 0.30.2 ``EulerDiscreteScheduler.set_timesteps``, also
+    used by the ancestral and LMS schedulers): ``sigma(t) = sqrt((1 - abar_t) / abar_t)`` interpolated at (possibly
+    non-integer) timesteps, a final sigma of 0 appended.  The sample lives in sigma space (``x = x_ddim / sqrt(abar_t)``);
+    the UNet sees ``x / sqrt(sigma^2 + 1)`` and the timestep ``float(np.float16(t))`` (pipeline.py:504-511).
+
+    ``timestep_spacing``: ``"linspace"`` (the default; what ``from_config`` yields for SD-1.x / 2.x configs, which have
+    no such key), ``"leading"`` (SDXL configs, with ``steps_offset``) or ``"trailing"``."""
+
+    SPACINGS = ("linspace", "leading", "trailing")
+
+    def __init__(self, num_inference_steps, timestep_spacing="linspace", steps_offset=1, **kw):
+        super().__init__(num_inference_steps, **kw)
+        if timestep_spacing not in self.SPACINGS:
+            raise ValueError(f"timestep_spacing must be one of {self.SPACINGS}, got {timestep_spacing!r}")
+        self.timestep_spacing = timestep_spacing
+        self.steps_offset = int(steps_offset)
+        n, n_train = self.n, self.n_train
+        if timestep_spacing == "linspace":
+            ts = np.linspace(0, n_train - 1, n, dtype=np.float32)[::-1].copy()
+        elif timestep_spacing == "leading":
+            ratio = n_train // n
+            ts = (np.arange(0, n) * ratio).round()[::-1].copy().astype(np.float32)
+            ts += np.float32(self.steps_offset)
+        else:
+            ratio = n_train / n
+            ts = np.arange(n_train, 0, -ratio).round().copy().astype(np.float32)
+            ts -= np.float32(1)
+        train_sigmas = np.sqrt((1.0 - self.abar) / self.abar)
+        self.raw_timesteps = ts
+        self.sigmas = np.concatenate([np.interp(ts.astype(np.float64), np.arange(n_train), train_sigmas), [0.0]])
+        smax = float(self.sigmas.max())
+        self.init_noise_sigma = smax if timestep_spacing in ("linspace", "trailing") else math.sqrt(smax * smax + 1.0)
+
+    @staticmethod
+    def c_in(sigma):
+        return 1.0 / math.sqrt(sigma * sigma + 1.0)
+
+    def scale_model_input(self, x, step_index):
+        return x * np.float32(self.c_in(self.sigmas[step_index]))
+
+    def first_in_scale(self, start=0):
+        return self.c_in(self.sigmas[start])
+
+    def add_noise(self, original_sample, noise, strength):
+        """x0 + sigma * noise at the start step (diffusers ``add_noise`` of the sigma schedulers)."""
+        s = np.float32(self.sigmas[self.start_step(strength)])
+        return original_sample + s * noise
+
+    def _step(self, i, j):
+        """Plan of absolute step ``i``, the ``j``-th step since the loop started (multistep state empty at j = 0)."""
+        raise NotImplementedError
+
+    def plan(self, start=0):
+        out = []
+        for j, i in enumerate(range(start, self.n)):
+            st = self._step(i, j)
+            st.timestep = float(np.float16(self.raw_timesteps[i]))
+            st.in_scale = self.c_in(self.sigmas[i + 1])
+            out.append(st)
+        return out
+
+
+class EulerDiscreteScheduler(_SigmaBase):
+    """diffusers 0.30.2 ``EulerDiscreteScheduler`` (epsilon prediction, s_churn = 0): ``x0 = x - sigma * eps``,
+    ``x_prev = x + (sigma_next - sigma) * eps``."""
+
+    def _step(self, i, j):
+        s, sn = self.sigmas[i], self.sigmas[i + 1]
+        return StepPlan(0.0, 1.0, sn - s, [0.0] * 4, 1.0, -s, [0.0] * 4)
+
+
+class EulerAncestralDiscreteScheduler(_SigmaBase):
+    """diffusers 0.30.2 ``EulerAncestralDiscreteScheduler`` (epsilon prediction): ``sigma_up = sqrt(sigma_next^2 *
+    (sigma^2 - sigma_next^2) / sigma^2)``, ``sigma_down = sqrt(sigma_next^2 - sigma_up^2)``,
+    ``x_prev = x + (sigma_down - sigma) * eps + sigma_up * z``."""
+
+    @property
+    def uses_noise(self):
+        return True
+
+    def _step(self, i, j):
+        s, sn = self.sigmas[i], self.sigmas[i + 1]
+        up = math.sqrt(sn * sn * (s * s - sn * sn) / (s * s))
+        down = math.sqrt(max(sn * sn - up * up, 0.0))
+        return StepPlan(0.0, 1.0, down - s, [0.0] * 4, 1.0, -s, [0.0] * 4, noise_scale=up, noise_draw=1 + j)
+
+
+def lms_coefficients(sigmas, i, order):
+    """c_k = integral from sigma_i to sigma_{i+1} of the Lagrange basis polynomial of node sigma_{i-k} over the nodes
+    sigma_i .. sigma_{i-order+1}, k = 0 .. order-1, in closed form (numpy.polynomial, float64).  The polynomials are
+    written in tau - sigma_i, so the integral is one evaluation at sigma_{i+1} - sigma_i without cancellation."""
+    from numpy.polynomial import polynomial as P
+    base = sigmas[i]
+    nodes = [sigmas[i - m] - base for m in range(order)]
+    out = []
+    for k in range(order):
+        p = np.array([1.0])
+        for m in range(order):
+            if m != k:
+                p = P.polymul(p, [-nodes[m], 1.0]) / (nodes[k] - nodes[m])
+        out.append(float(P.polyval(sigmas[i + 1] - base, P.polyint(p))))
+    return out
+
+
+class LMSDiscreteScheduler(_SigmaBase):
+    """diffusers 0.30.2 ``LMSDiscreteScheduler`` (order 4, epsilon prediction): ``x_prev = x + sum_k c_k eps_{i-k}``,
+    ``order = min(steps so far + 1, 4)``, ``c_k`` from ``lms_coefficients``.  The derivative ``(x - x0) / sigma`` is
+    ``eps`` itself, so the history ring holds past eps: step ``j`` since the start pushes to slot ``j % 3``."""
+    order = 4
+
+    def _step(self, i, j):
+        order = min(j + 1, self.order)
+        c = lms_coefficients(self.sigmas, i, order)
+        ch = [0.0] * 4
+        for k in range(1, order):
+            ch[(j - k) % 3] = c[k]
+        return StepPlan(0.0, 1.0, c[0], ch, 1.0, -self.sigmas[i], [0.0] * 4, n_hist=3 if order > 1 else 0,
+                        push_eps_slot=j % 3)
+
+
 SCHEDULER_MAP = {
     "DDIM": DDIMScheduler,
     "DPMSolverMultistep": DPMSolverMultistepScheduler,
+    "EulerAncestralDiscrete": EulerAncestralDiscreteScheduler,
+    "EulerDiscrete": EulerDiscreteScheduler,
+    "LMSDiscrete": LMSDiscreteScheduler,
     "PNDM": PNDMScheduler,
 }
 
@@ -259,18 +416,25 @@ def make_scheduler(name, num_inference_steps, **kw):
     return SCHEDULER_MAP[name](num_inference_steps, **kw)
 
 
-def apply_plan_host(step: StepPlan, guidance, eps_uncond, eps_text, x, hist):
-    """numpy mirror of the device kernel's arithmetic (host-logic tests only)."""
+def apply_plan_host(step: StepPlan, guidance, eps_uncond, eps_text, x, hist, noise=None, return_unet_in=False):
+    """numpy mirror of the device kernel's arithmetic (host-logic tests only).  ``noise``: the step's normals (needed
+    when ``step.noise_scale != 0``); ``return_unet_in``: also return the next UNet input ``in_scale * x_prev``."""
     eps = eps_uncond + guidance * (eps_text - eps_uncond)
     xp = step.cx * x + step.ce * eps
     x0 = step.x0_cx * x + step.x0_ce * eps
     for j in range(step.n_hist):
         xp = xp + step.ch[j] * hist[j]
         x0 = x0 + step.x0_ch[j] * hist[j]
+    if step.noise_scale != 0.0:
+        if noise is None:
+            raise ValueError("this step adds noise: pass `noise`")
+        xp = xp + step.noise_scale * noise
     if step.push_eps_slot >= 0:
         hist[step.push_eps_slot] = eps
     if step.push_x0_slot >= 0:
         hist[step.push_x0_slot] = x0
     if step.push_x_slot >= 0:
         hist[step.push_x_slot] = x
+    if return_unet_in:
+        return xp, x0, step.in_scale * xp
     return xp, x0
